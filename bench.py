@@ -66,7 +66,32 @@ def parse():
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary BASELINE configs / reference-on-GPU legs")
     ap.add_argument("--workload", default="metric", choices=["metric", "config4"],
                     help="metric = BASELINE.json's metric workload (default); config4 = 512^3 -> 1024^2, 256 poses sharded over the GPUs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0's shard) as DIR/<name>.npy, float32, at most 64 MB in all")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, arrays):
+    """Saves each tensor of `arrays` as out_dir/<name>.npy in float32.  When together they exceed DUMP_BYTES, every tensor
+    keeps the same fraction of its elements, flattened, at positions drawn from a fixed seed: the positions depend only on
+    the tensor sizes, so two builds of the project run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(4 * t.numel() for t in arrays.values())
+    keep = min(1.0, (DUMP_BYTES - 1024 * len(arrays)) / total)  # 1 KB per file for the .npy header
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if keep < 1.0:
+            flat = t.reshape(-1)
+            n = max(1, int(flat.numel() * keep))
+            pos = torch.randint(flat.numel(), (n,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = flat[pos.to(flat.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 def hbm_peak():
@@ -731,6 +756,10 @@ def run_ours(args, rank, local_rank, world):
         t_end.record(stream)
         barrier()
     ms_total = t_start.elapsed_time(t_end)
+    if args.dump_outputs and rank == 0:  # the legs below overwrite these buffers
+        last = outs[(state["k"] - 1) & 1] if world > 1 else outs[0]
+        dump = {"image": last.reshape(B, 1, args.det, args.det).cpu(), "grad_source": g_src.cpu(),
+                "grad_target": g_tgt.cpu(), "grad_raylen": g_len.cpu()}
     sens_list = [e[0].elapsed_time(e[1]) for e in events]
     sens_bwd_list = [e[1].elapsed_time(e[2]) for e in events]
     sens_ms = float(np.mean(sens_list))
@@ -849,6 +878,9 @@ def run_ours(args, rank, local_rank, world):
             e2e_ms_total, e2e_mode = g_start.elapsed_time(g_end), "cuda-graph replay of the public-API step"
         except Exception as exc:  # capture is an optimisation of the launch path only; never hide the eager number
             e2e_mode = f"eager (graph capture failed: {type(exc).__name__})"
+    if args.dump_outputs and rank == 0:  # + what the last end-to-end step handed back to the host
+        dump.update(e2e_image=img_h, e2e_grad_rot=grad_h[0], e2e_grad_xyz=grad_h[1], e2e_loss=loss_h)
+        dump_outputs(args.dump_outputs, dump)
 
     # ---- max over ranks -------------------------------------------------------------------------------------
     stats = torch.tensor([ms_total, e2e_ms_total, fwd_ms, bwd_ms, e2e_eager_ms_total, sens_ms, sens_bwd_ms], device=dev,
@@ -1035,6 +1067,8 @@ def run_config4(args, rank, local_rank, world):
         e1.record()
         barrier()
     ms_total = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:  # before the kernel timings below overwrite `out`
+        dump_outputs(args.dump_outputs, {"image": out.reshape(B, 1, det, det)})
     t_brick = _time_events(brick, 3, warmup=1)
     t_slab = _time_events(slab, 3, warmup=1)
     stats = torch.tensor([ms_total, float(np.median(t_brick)), float(np.median(t_slab)), float(visits)], device=dev, dtype=torch.float64)

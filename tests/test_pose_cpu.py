@@ -1,13 +1,13 @@
-"""Host-side pose algebra (diffdrr_b200/pose.py) against the UNMODIFIED reference (diffdrr/pose.py), when it is available
-(build container; /root/reference or baseline/_ref), plus round trips that hold anywhere: all nine parameterisations in
-BOTH directions (ADVICE r1: se3_log_map / quaternion_adjugate / rotation_10d were missing from RigidTransform.convert)."""
+"""Host-side pose algebra (diffdrr_b200/pose.py) against the UNMODIFIED reference (diffdrr/pose.py), recorded in
+tests/golden/pose_reference.npz by make_golden_pose.py, plus round trips: all nine parameterisations in BOTH directions
+(se3_log_map / quaternion_adjugate / rotation_10d included in RigidTransform.convert)."""
 import os
-import sys
 
+import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT
+from conftest import GOLDEN
 from diffdrr_b200.pose import PARAMETERIZATIONS, RigidTransform, convert
 
 
@@ -27,32 +27,20 @@ def test_convert_round_trip(param):
     assert torch.allclose(again.matrix, pose.matrix, atol=2e-4, rtol=1e-5), param
 
 
-def _reference_pose_module():
-    for base in ("/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if os.path.isdir(os.path.join(base, "diffdrr")):
-            for p in (os.path.join(ROOT, "tests", "_refshim"), base):
-                if p not in sys.path:
-                    sys.path.insert(0, p)
-            try:
-                import diffdrr.pose as ref
-                return ref
-            except Exception:
-                return None
-    return None
+@pytest.fixture(scope="module")
+def ref():
+    return {k: torch.from_numpy(v) for k, v in np.load(os.path.join(GOLDEN, "pose_reference.npz")).items()}
 
 
 @pytest.mark.parametrize("param", [p for p in PARAMETERIZATIONS if p != "matrix"])
-def test_convert_matches_the_reference_both_ways(param):
-    ref = _reference_pose_module()
-    if ref is None:
-        pytest.skip("reference sources not available on this box")
-    pose = _poses(seed=3)
+def test_convert_matches_the_reference_both_ways(param, ref):
+    pose = RigidTransform(ref["matrix"].clone())
     kw = dict(convention="ZXY") if param == "euler_angles" else {}
     ours = pose.convert(param, **kw)
-    theirs = ref.RigidTransform(pose.matrix.clone()).convert(param, **kw)
+    theirs = [ref[f"{param}_{i}"] for i in range(int(ref[f"{param}_n"]))]
+    assert len(ours) == len(theirs), param
     for a, b in zip(ours, theirs):
         assert torch.allclose(a, b, atol=5e-4, rtol=1e-4), param
     fwd_ours = convert(*theirs, parameterization=param, **kw).matrix
-    fwd_ref = ref.convert(*theirs, parameterization=param, **kw).matrix
-    assert torch.allclose(fwd_ours, fwd_ref, atol=5e-4, rtol=1e-4), param
-    assert torch.allclose(pose.get_se3_log(), ref.RigidTransform(pose.matrix.clone()).get_se3_log(), atol=5e-4, rtol=1e-4)
+    assert torch.allclose(fwd_ours, ref[f"{param}_fwd"], atol=5e-4, rtol=1e-4), param
+    assert torch.allclose(pose.get_se3_log(), ref["se3_log"], atol=5e-4, rtol=1e-4)
