@@ -55,6 +55,48 @@ B200_HD float add_rn(float a, float b)
 #endif
 }
 
+// A pair of floats updated by one packed f32x2 instruction on sm_100a (FADD2 / FMUL2 / FFMA2: both lanes rounded exactly
+// as the scalar add.rn / mul.rn / fma.rn); two scalar operations in the host emulation, which is compiled without contraction.
+#if defined(__CUDACC__)
+using Pair = float2;
+#else
+struct Pair {
+    float x, y;
+};
+#endif
+B200_HD Pair add2_rn(Pair a, Pair b)
+{
+#if defined(__CUDA_ARCH__)
+    return __fadd2_rn(a, b);
+#else
+    return Pair{a.x + b.x, a.y + b.y};
+#endif
+}
+B200_HD Pair sub2_rn(Pair a, Pair b)
+{
+#if defined(__CUDA_ARCH__)
+    return __fadd2_rn(a, make_float2(-b.x, -b.y));
+#else
+    return Pair{a.x - b.x, a.y - b.y};
+#endif
+}
+B200_HD Pair mul2_rn(Pair a, Pair b)
+{
+#if defined(__CUDA_ARCH__)
+    return __fmul2_rn(a, b);
+#else
+    return Pair{a.x * b.x, a.y * b.y};
+#endif
+}
+B200_HD Pair fma2_rn(Pair a, Pair b, Pair c)
+{
+#if defined(__CUDA_ARCH__)
+    return __ffma2_rn(a, b, c);
+#else
+    return Pair{fmaf(a.x, b.x, c.x), fmaf(a.y, b.y, c.y)};
+#endif
+}
+
 // accumulate into the volume gradient: red.global.add.f32 on the device, plain add in the host emulation
 B200_HD void red_add(float* addr, float v)
 {

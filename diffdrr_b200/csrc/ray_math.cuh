@@ -889,74 +889,132 @@ struct MinorAxes {
     B200_HD static int local(int axis) { return axis == U ? 0 : (axis == V ? 1 : 2); }
 };
 
-// lean_step_ax with the crossing reported as a LOCAL index of MinorAxes<M>; same sequential tie order (lowest axis
-// first).  If the minimum is below the exit alpha and neither axis 0 nor axis 1 attains it, axis 2 does -- no third compare.
-#define B200_LEAN_STEP_UV_ASM(PV, PU)                                                                                  \
-    asm("{\n\t"                                                                                                    \
-        ".reg .pred q, p0, p1, p2;\n\t"                                                                             \
-        ".reg .f32 nx;\n\t"                                                                                         \
-        "min.f32 nx, %0, %1, %2;\n\t"                                                                               \
-        "sub.f32 %8, nx, %6;\n\t"                                                                                   \
-        "mov.f32 %6, nx;\n\t"                                                                                       \
-        "setp.lt.f32 q, nx, %10;\n\t"                                                                               \
-        "setp.eq.and.f32 p0, %0, nx, q;\n\t"                                                                        \
-        "setp.eq.and.f32 p1, %1, nx, q;\n\t"                                                                        \
-        "and.pred p1, p1, !p0;\n\t"                                                                                 \
-        "or.pred p2, p0, p1;\n\t"                                                                                   \
-        "and.pred p2, q, !p2;\n\t"                                                                                  \
-        "selp.s32 %9, 1, 2, " PV ";\n\t"                                                                            \
-        "selp.s32 %9, 0, %9, " PU ";\n\t"                                                                           \
-        "@p0 add.f32 %3, %3, 0f3F800000;\n\t"                                                                       \
-        "@p1 add.f32 %4, %4, 0f3F800000;\n\t"                                                                       \
-        "@p2 add.f32 %5, %5, 0f3F800000;\n\t"                                                                       \
-        "@p0 fma.rn.f32 %0, %3, %11, %14;\n\t"                                                                      \
-        "@p1 fma.rn.f32 %1, %4, %12, %15;\n\t"                                                                      \
-        "@p2 fma.rn.f32 %2, %5, %13, %16;\n\t"                                                                      \
-        "@p0 add.s32 %7, %7, %17;\n\t"                                                                              \
-        "@p1 add.s32 %7, %7, %18;\n\t"                                                                              \
-        "@p2 add.s32 %7, %7, %19;\n\t"                                                                              \
-        "}"                                                                                                         \
-        : "+f"(s.an0), "+f"(s.an1), "+f"(s.an2), "+f"(s.nf0), "+f"(s.nf1), "+f"(s.nf2), "+f"(s.acur), "+r"(s.off),  \
-          "=f"(len), "=r"(ax)                                                                                       \
-        : "f"(k.a_out), "f"(k.da0), "f"(k.da1), "f"(k.da2), "f"(k.a00), "f"(k.a01), "f"(k.a02), "r"(k.so0),         \
-          "r"(k.so1), "r"(k.so2))
+// The sensitivities walk's state: lean_step_ax's (an, nf, acur, off) with the two MINOR axes' alphas and counters held as
+// pairs (u, v), so that one packed f32x2 instruction updates both (FADD2 / FFMA2 on sm_100a).
+struct SensState {
+    Pair an_uv, nf_uv;  // minor axes
+    float an_m, nf_m;   // major axis
+    float acur;
+    int off;
+};
+struct SensConst {
+    Pair da_uv, a0_uv;
+    float da_m, a0_m, a_out;
+    int so0, so1, so2;
+};
+
+// |1/d| of the minor axes as a pair of their own.  Left alone, the compiler folds them into an |abs| modifier on the 1/d
+// registers the ray keeps for after the walk; for major axes 1 and 2 those are not adjacent and every FFMA2 of the walk
+// would first copy them into a register pair.  (x + 0 is x here: |1/d| is never -0.)
+B200_HD Pair own_pair(float a, float b)
+{
+#if defined(__CUDA_ARCH__)
+    float ra, rb;
+    asm("add.rn.f32 %0, %1, 0f00000000;" : "=f"(ra) : "f"(a));
+    asm("add.rn.f32 %0, %1, 0f00000000;" : "=f"(rb) : "f"(b));
+    return Pair{ra, rb};
+#else
+    return Pair{a, b};
+#endif
+}
 
 template <int M>
-B200_HD float lean_step_uv(LeanState& s, const LeanConst& k, int& ax)
+B200_HD void sens_init(const Walk& w, int st0, int st1, int st2, SensState& s, SensConst& k)
 {
-    float len;
-#if defined(__CUDA_ARCH__)
-    if (M == 0) B200_LEAN_STEP_UV_ASM("p2", "p1");       // minor axes (1, 2)
-    else if (M == 1) B200_LEAN_STEP_UV_ASM("p2", "p0");  // minor axes (0, 2)
-    else B200_LEAN_STEP_UV_ASM("p1", "p0");              // minor axes (0, 1)
-#else
-    int axis;
-    len = lean_step_ax(s, k, axis);
-    ax = MinorAxes<M>::local(axis);
-#endif
-    return len;
+    using Ax = MinorAxes<M>;
+    k.da_uv = own_pair(w.da[Ax::U], w.da[Ax::V]);
+    k.a0_uv = Pair{w.a0[Ax::U], w.a0[Ax::V]};
+    k.da_m = w.da[M];
+    k.a0_m = w.a0[M];
+    k.a_out = w.a_out;
+    k.so0 = w.sti[0] * st0; k.so1 = w.sti[1] * st1; k.so2 = w.sti[2] * st2;
+    s.an_uv = Pair{w.an[Ax::U], w.an[Ax::V]};
+    s.nf_uv = Pair{w.nf[Ax::U], w.nf[Ax::V]};
+    s.an_m = w.an[M];
+    s.nf_m = w.nf[M];
+    s.acur = w.hit ? w.a_in : w.a_out;
+    s.off = w.idx[0] * st0 + w.idx[1] * st1 + w.idx[2] * st2;
 }
 
-// Au += coef*alpha, Cu += coef for LOCAL index 0; (Av, Cv) for 1; nothing for 2.
-B200_HD void minor_accumulate(int ax, float coef, float alpha, float& Au, float& Av, float& Cu, float& Cv)
+// alpha of the next plane on global axis A
+template <int M, int A>
+B200_HD float sens_an(const SensState& s)
+{
+    return A == M ? s.an_m : (A == MinorAxes<M>::U ? s.an_uv.x : s.an_uv.y);
+}
+// crossing counter of global axis A
+template <int M, int A>
+B200_HD float sens_nf(const SensState& s)
+{
+    return A == M ? s.nf_m : (A == MinorAxes<M>::U ? s.nf_uv.x : s.nf_uv.y);
+}
+
+// One step of the sensitivities walk: lean_step_ax's crossing -- the same alphas and the same sequential tie order (lowest
+// axis first; nothing is crossed at the exit alpha) -- with the crossed axis reported as the mask pair m = (crossed u,
+// crossed v) in {0, 1}^2 ((0, 0): the major axis or no crossing).  The minor axes are updated without a predicate:
+// nf_uv += m, an_uv = fma(nf_uv, da_uv, a0_uv) recomputes an unchanged alpha bit for bit (the walk's set-up forms every `an`
+// by that same expression), up to the sign of a zero counter.  Ties:
+//   q = nx < a_out;   p0 = q & (an0 == nx), x = q & !(an0 == nx);   p1 = x & (an1 == nx), p2 = x & !(an1 == nx)
+// (when q holds and neither axis 0 nor 1 attains the minimum, axis 2 does; `neu` is !(==) also for a NaN alpha).
+// sm_100a: FMNMX3, 5 FSETP, 2 FSEL, predicated FADD + FFMA (major), FADD2 + FFMA2 (minor), 3 predicated IADD (one of them
+// as IADD + SEL).
+#define B200_SENS_STEP_ASM(PM, PU, PV)                                                                                 \
+    asm("{\n\t"                                                                                                    \
+        ".reg .pred q, x, p0, p1, p2;\n\t"                                                                          \
+        ".reg .f32 nx;\n\t"                                                                                         \
+        "min.f32 nx, %6, %7, %8;\n\t"                                                                               \
+        "mov.f32 %2, nx;\n\t"                                                                                       \
+        "setp.lt.f32 q, nx, %9;\n\t"                                                                               \
+        "setp.eq.and.f32 p0, %6, nx, q;\n\t"                                                                        \
+        "setp.neu.and.f32 x, %6, nx, q;\n\t"                                                                        \
+        "setp.eq.and.f32 p1, %7, nx, x;\n\t"                                                                        \
+        "setp.neu.and.f32 p2, %7, nx, x;\n\t"                                                                       \
+        "selp.f32 %4, 0f3F800000, 0f00000000, " PU ";\n\t"                                                          \
+        "selp.f32 %5, 0f3F800000, 0f00000000, " PV ";\n\t"                                                          \
+        "@" PM " add.rn.f32 %1, %1, 0f3F800000;\n\t"                                                                \
+        "@" PM " fma.rn.f32 %0, %1, %10, %11;\n\t"                                                                  \
+        "@p2 add.s32 %3, %3, %14;\n\t"                                                                              \
+        "@p1 add.s32 %3, %3, %13;\n\t"                                                                              \
+        "@p0 add.s32 %3, %3, %12;\n\t"                                                                              \
+        "}"                                                                                                         \
+        : "+f"(s.an_m), "+f"(s.nf_m), "=f"(s.acur), "+r"(s.off), "=f"(m.x), "=f"(m.y)                                 \
+        : "f"(sens_an<M, 0>(s)), "f"(sens_an<M, 1>(s)), "f"(sens_an<M, 2>(s)), "f"(k.a_out), "f"(k.da_m), "f"(k.a0_m), \
+          "r"(k.so0), "r"(k.so1), "r"(k.so2))
+
+template <int M>
+B200_HD void sens_step(SensState& s, const SensConst& k, Pair& m)
 {
 #if defined(__CUDA_ARCH__)
-    asm("{\n\t"
-        ".reg .pred q0, q1;\n\t"
-        "setp.eq.s32 q0, %4, 0;\n\t"
-        "setp.eq.s32 q1, %4, 1;\n\t"
-        "@q0 fma.rn.f32 %0, %5, %6, %0;\n\t"
-        "@q1 fma.rn.f32 %1, %5, %6, %1;\n\t"
-        "@q0 add.f32 %2, %2, %5;\n\t"
-        "@q1 add.f32 %3, %3, %5;\n\t"
-        "}"
-        : "+f"(Au), "+f"(Av), "+f"(Cu), "+f"(Cv)
-        : "r"(ax), "f"(coef), "f"(alpha));
+    if (M == 0) B200_SENS_STEP_ASM("p0", "p1", "p2");       // minor axes (1, 2)
+    else if (M == 1) B200_SENS_STEP_ASM("p1", "p0", "p2");  // minor axes (0, 2)
+    else B200_SENS_STEP_ASM("p2", "p0", "p1");              // minor axes (0, 1)
 #else
-    if (ax == 0) { Au = fmaf(coef, alpha, Au); Cu += coef; }
-    if (ax == 1) { Av = fmaf(coef, alpha, Av); Cv += coef; }
+    const float a0 = sens_an<M, 0>(s), a1 = sens_an<M, 1>(s), a2 = sens_an<M, 2>(s);
+    const float nx = fminf(fminf(a0, a1), a2);
+    s.acur = nx;
+    const bool q = nx < k.a_out;
+    const bool p[3] = {q && a0 == nx, q && !(a0 == nx) && a1 == nx, q && !(a0 == nx) && !(a1 == nx)};
+    m = Pair{p[MinorAxes<M>::U] ? 1.0f : 0.0f, p[MinorAxes<M>::V] ? 1.0f : 0.0f};
+    if (p[M]) { s.nf_m += 1.0f; s.an_m = fmaf(s.nf_m, k.da_m, k.a0_m); }
+    if (p[0]) s.off += k.so0;
+    if (p[1]) s.off += k.so1;
+    if (p[2]) s.off += k.so2;
 #endif
+    s.nf_uv = add2_rn(s.nf_uv, m);
+    s.an_uv = fma2_rn(s.nf_uv, k.da_uv, k.a0_uv);
 }
+
+// (Au, Av) += coef*alpha * m, (Cu, Cv) += coef * m: the crossing's coefficient goes to the minor axis its mask selects; the
+// other one gets an exact 0 added (FMUL2, FFMA2, FADD2).
+B200_HD void minor_accumulate(Pair m, float coef, float alpha, Pair& A, Pair& C)
+{
+    const Pair cm = mul2_rn(m, Pair{coef, coef});
+    A = fma2_rn(cm, Pair{alpha, alpha}, A);
+    C = add2_rn(C, cm);
+}
+
+// mask pair of a LOCAL index of MinorAxes<M> (0 = u, 1 = v, 2 = neither)
+B200_HD Pair minor_mask(int local) { return Pair{local == 0 ? 1.0f : 0.0f, local == 1 ? 1.0f : 0.0f}; }
 
 // How the sensitivities walk fetches its voxels: one scalar load per visit from the volume as stored (production), or --
 // EXPERIMENT, see siddon_ray_lean_box_chunk -- W-voxel chunks from a major-axis-fastest copy, re-used across visits.
@@ -1006,63 +1064,67 @@ B200_HD float siddon_ray_sens_box_m(const float* vol, const VolDims& dims, const
     Load loader;
     const Walk w = start_walk_frame<CUT>(ray, dims, lo_v, hi_v, shift);
     if (!w.hit) return 0.0f;
-    LeanConst k;
-    LeanState s;
-    lean_init(w, st0, st1, st2, s, k);
-    float Au = 0.0f, Av = 0.0f, Cu = 0.0f, Cv = 0.0f;
-    float acc = 0.0f, vprev = 0.0f, aprev = w.a_in;
-    int axprev = Ax::local(w.entry_axis);
-    const bool any = s.acur < k.a_out;  // false: the box is only touched (a_in == a_out)
+    SensConst k;
+    SensState s;
+    sens_init<M>(w, st0, st1, st2, s, k);
+    Pair Auv = {0.0f, 0.0f}, Cuv = {0.0f, 0.0f};
+    float acc = 0.0f;
+    Pair prev = {0.0f, w.a_in};  // (value of the voxel before, alpha of the crossing that left it)
+    Pair mprev = minor_mask(Ax::local(w.entry_axis));
+    if (!(s.acur < k.a_out)) {  // the box is only touched (a_in == a_out): the entry crossing leads into the one voxel
+        prev.x = loader.at(vol, s.off);
+        minor_accumulate(mprev, -prev.x, w.a_in, Auv, Cuv);
+    }
     while (s.acur < k.a_out) {
-        float aend[U], v[U];
-        int offs[U], ax[U];
+        float v[U];
+        int offs[U];
+        Pair m[U], va[U];
 #pragma unroll
         for (int j = 0; j < U; ++j) {
             offs[j] = s.off;
-            (void)lean_step_uv<M>(s, k, ax[j]);
-            aend[j] = s.acur;
+            sens_step<M>(s, k, m[j]);
+            va[j].y = s.acur;
         }
         loader.template batch<U>(vol, offs, v);
 #pragma unroll
         for (int j = 0; j < U; ++j) {
-            // crossing (axprev, aprev) led into voxel j; padding steps after the exit carry local index 2 and length 0.
-            // The segment length is re-formed from the two alphas (same subtraction the step did) instead of being kept
-            // in a register across the loads: U fewer live registers.
-            minor_accumulate(axprev, vprev - v[j], aprev, Au, Av, Cu, Cv);
-            acc = fmaf(aend[j] - aprev, v[j], acc);
-            vprev = v[j];
-            axprev = ax[j];
-            aprev = aend[j];
+            // crossing (mprev, prev.y) led into voxel j; padding steps after the exit carry the mask (0, 0) and length 0.
+            // One FADD2 forms (v_j - v_before, alpha_j - alpha_before) = (-coef, segment length): the same two
+            // subtractions, the first with its operands swapped, which negates it exactly.
+            va[j].x = v[j];
+            const Pair d = sub2_rn(va[j], prev);
+            minor_accumulate(mprev, -d.x, prev.y, Auv, Cuv);
+            acc = fmaf(d.y, va[j].x, acc);
+            prev = va[j];
+            mprev = m[j];
         }
     }
-    if (!any) {
-        const float v0 = loader.at(vol, s.off);
-        minor_accumulate(Ax::local(w.entry_axis), -v0, w.a_in, Au, Av, Cu, Cv);
-        vprev = v0;
-    }
+    float vprev = prev.x;
     // Tail: identical to siddon_ray_bwd_lean_box (ties with the exit alpha, lowest axis first)
     int ax_exit = 3;
     {
-        const bool t0 = s.an0 <= k.a_out, t1 = s.an1 <= k.a_out, t2 = s.an2 <= k.a_out;
-        const bool b0 = s.nf0 == w.nx[0], b1 = s.nf1 == w.nx[1], b2 = s.nf2 == w.nx[2];
+        const float an0 = sens_an<M, 0>(s), an1 = sens_an<M, 1>(s), an2 = sens_an<M, 2>(s);
+        const bool t0 = an0 <= k.a_out, t1 = an1 <= k.a_out, t2 = an2 <= k.a_out;
+        const bool b0 = sens_nf<M, 0>(s) == w.nx[0], b1 = sens_nf<M, 1>(s) == w.nx[1], b2 = sens_nf<M, 2>(s) == w.nx[2];
         if (t0 && b0) ax_exit = 0;
         if (ax_exit == 3 && t0) {
             s.off += k.so0;
             const float vm = loader.at(vol, s.off);
-            minor_accumulate(Ax::local(0), vprev - vm, k.a_out, Au, Av, Cu, Cv);
+            minor_accumulate(minor_mask(Ax::local(0)), vprev - vm, k.a_out, Auv, Cuv);
             vprev = vm;
         }
         if (ax_exit == 3 && t1 && b1) ax_exit = 1;
         if (ax_exit == 3 && t1) {
             s.off += k.so1;
             const float vm = loader.at(vol, s.off);
-            minor_accumulate(Ax::local(1), vprev - vm, k.a_out, Au, Av, Cu, Cv);
+            minor_accumulate(minor_mask(Ax::local(1)), vprev - vm, k.a_out, Auv, Cuv);
             vprev = vm;
         }
         if (ax_exit == 3 && t2 && b2) ax_exit = 2;
-        if (ax_exit == 3) ax_exit = (s.an0 <= s.an1 && s.an0 <= s.an2) ? 0 : (s.an1 <= s.an2 ? 1 : 2);
+        if (ax_exit == 3) ax_exit = (an0 <= an1 && an0 <= an2) ? 0 : (an1 <= an2 ? 1 : 2);
     }
-    minor_accumulate(Ax::local(ax_exit), vprev, k.a_out, Au, Av, Cu, Cv);
+    minor_accumulate(minor_mask(Ax::local(ax_exit)), vprev, k.a_out, Auv, Cuv);
+    const float Au = Auv.x, Av = Auv.y, Cu = Cuv.x, Cv = Cuv.y;
     A[Ax::U] += Au;
     A[Ax::V] += Av;
     A[M] += acc - Au - Av;  // sum_a A_a = sum_j v_j len_j over the box

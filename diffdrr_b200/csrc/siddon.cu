@@ -739,7 +739,9 @@ cudaError_t launch_x_siddon_sens_chunk(const float* volT, VolDims dims, int axis
 //   forward   B = 1: 187 (32-plane slabs) -> 95 (K = 12);  2: 250 -> 152;  4: 365 -> 248;  8: 601 (brick 591) -> 504;
 //             16: 1142 (brick 1099) -> 1032 (K = 16)  -- the fastest forward kernel at every batch size measured (41 % of HBM roofline)
 //   sens      B = 1: 193 (thread per ray) -> 115 (K = 8..16);  2: 281 -> 192;  4: 394 (96-plane slabs) -> 312;  8: 637 (48-plane
-//             slabs) -> 639;  16: 1243 -> 1273  -- the slab-major kernel keeps batches >= 8 (its volume re-use through L2 pays there)
+//             slabs) -> 639;  16: 1243 -> 1273  -- the slab-major kernel keeps batches >= 8 (its volume re-use through L2 pays there).
+//             Re-measured at 16 poses with the packed-pair sensitivities step (profiles/r03_tune_sens_routing.log, 3 runs): 48-plane
+//             slabs 1182-1191, pieces K = 8 / 12 / 16: 1260-1309 / 1254-1311 / 1288-1321 -- the slabs still win
 // `load` = B * H * W in units of 256^2 rays.  Pieces thinner than ~24 planes only add set-up; volumes below 384^3 were not measured
 // at batch sizes > 4 (the slab-major tuning of BASELINE config 2 stands there), volumes below 96 voxels keep one thread per ray.
 // Returns K, 0 = not used.
